@@ -241,6 +241,25 @@ def run_reference_arm(args, wl, rank):
 
 
 # ------------------------------------------------------------------------------------
+DUMP_USERS = 1024   # assign0 is dumped for a fixed, seeded sample of this many users (all frames)
+
+
+def dump_outputs(torch, out_dir, sp, tr=None):
+    """Writes the outputs of one step as out_dir/<name>.npy so that two builds can be compared output for output:
+    the per-frame rows whole, assign0 [F,U] for DUMP_USERS users drawn with a fixed seed (their indices in
+    assign0_users.npy).  Integer outputs are written as float32 (uint16 tile ids) or float64 (int32 counts), exactly."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    U = sp.assign0.shape[1]
+    users = np.sort(np.random.default_rng(0).choice(U, size=min(U, DUMP_USERS), replace=False))
+    idx = torch.from_numpy(users).to(sp.assign0.device)
+    arrays = {"entropy": sp.entropy.double(), "hist0": sp.hist0.double(),
+              "assign0": sp.assign0.index_select(1, idx).float(), "assign0_users": torch.from_numpy(users).double()}
+    if tr is not None:
+        arrays.update(tr_entropy=tr.entropy.double(), tr_prev_count0=tr.prev_count0.double())
+    for name, t in arrays.items():
+        np.save(out_dir / f"{name}.npy", t.cpu().numpy())
+
+
 def time_steps(torch, fn, steps, warmup):
     """ms per call of fn: CUDA events on the current stream, synchronised on both sides."""
     for _ in range(warmup):
@@ -339,7 +358,13 @@ def main():
     ap.add_argument("--sustained-seconds", type=float, default=2.0)
     ap.add_argument("--gather-hist0", action="store_true",
                     help="N > 1: also all-gather the hist0[F,T0] rows (5.8 MB per rank), not only entropy[F]")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, float32/float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -406,6 +431,7 @@ def main():
     pending = [[] for _ in outs]
     out = outs[0]
     counter = [0]
+    last = [None]   # what the most recent step returned
 
     def drain(slot):
         for w in pending[slot]:
@@ -417,10 +443,11 @@ def main():
         counter[0] += 1
         drain(slot)  # the all-gather that last read this slot's buffers
         o = outs[slot]
+        last[0] = None  # released before the call, so that its memory is reused as before
         if args.transition:  # both analyzers in one pass over the input (configs[4])
-            eng.analyze(packed, want_per_k=False, want_pairs0=False)
+            last[0] = eng.analyze(packed, want_per_k=False, want_pairs0=False)
         else:
-            eng.spatial(packed, out=o)
+            last[0] = (eng.spatial(packed, out=o), None)
         if world > 1:  # the path's only exchange: the all-gather of the per-frame results
             pending[slot] = [dist.all_gather_into_tensor(gathered[slot][0], o.entropy, async_op=True)]
             if args.gather_hist0:  # hist0 / assign0 normally stay on the rank that owns the frames
@@ -462,6 +489,8 @@ def main():
     ms = ev0.elapsed_time(ev1)
     launches = eng.launch_count() - launches0
     replays = eng.graph_replays() - replays0
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(torch, args.dump_outputs, *last[0])
     # per-kernel device times: the SAME steps once more with an event pair around every launch (the library then
     # launches kernel by kernel instead of replaying its graph), right after the timed region
     eng.profile(True)
@@ -612,8 +641,8 @@ def main():
     # secondary workloads (not the headline), device-resident
     extra = {}
     if rank == 0 and world == 1 and not args.no_extra and args.workload == "c3":
-        def timed_spatial(e2, p2, o2, n=5):
-            return time_steps(torch, lambda: e2.spatial(p2, out=o2), n, 3)
+        def timed_spatial(e2, p2, o2):
+            return time_steps(torch, lambda: e2.spatial(p2, out=o2), args.steps, 3)
 
         def outs_for(e2, F2, U2):
             return SpatialResult(entropy=torch.empty(F2, dtype=torch.float64, device=device), per_k=None,
@@ -632,7 +661,7 @@ def main():
                            "whole_step_frac": ALG_BYTES_PER_SAMPLE * rate / 1e9 / peak_gbs}
             if name == "c5shard":
                 # configs[4] asks for weighted spatial AND transition entropy: both analyzers in one pass (vet_analyze)
-                ms3 = time_steps(torch, lambda: e2.analyze(p2, want_per_k=False, want_assign0=True, want_pairs0=False), 5, 4)
+                ms3 = time_steps(torch, lambda: e2.analyze(p2, want_per_k=False, want_assign0=True, want_pairs0=False), args.steps, 4)
                 extra["c5shard_analyze"] = {"workload": w2["desc"] + " + transition entropy, one pass over the input",
                                             "ms_per_step": ms3, "value": w2["F"] * w2["U"] / (ms3 * 1e-3), "unit": UNIT,
                                             "whole_step_frac": ALG_BYTES_PER_SAMPLE * w2["F"] * w2["U"] / (ms3 * 1e-3) / 1e9 / peak_gbs}
@@ -653,7 +682,7 @@ def main():
         # configs[3]: transition-entropy matrices for tile_counts=[200,500,1000] on the headline tensor shape
         p4 = synth_on_device(torch, 3600, 100_000, 20260000 + 4000, device)
         e4 = get_engine(100, 200, [200, 500, 1000], EntropyConfig(use_weight_distribution=False), device)
-        ms4 = time_steps(torch, lambda: e4.transition(p4, want_pairs0=False, want_per_k=False), 5, 4)
+        ms4 = time_steps(torch, lambda: e4.transition(p4, want_pairs0=False, want_per_k=False), args.steps, 4)
         extra["c4"] = {"workload": "configs[3]: synthetic 100k users x 3600 frames, tile_counts=[200,500,1000], transition entropy",
                        "ms_per_step": ms4, "value": 3599 * 100_000 / (ms4 * 1e-3), "unit": "user frame pairs/s (each under 3 tile counts)",
                        "roofline_ms": ALG_BYTES_PER_SAMPLE * 3600 * 100_000 / (peak_gbs * 1e9) * 1e3}
@@ -663,7 +692,7 @@ def main():
     # configs[4], frame-sharded over the ranks of this run: at EVERY N, all ranks
     if not args.no_c5 and args.workload == "c3":
         extra["c5_sharded"] = c5_sharded(torch, dist, device, rank, world, local_rank, peak_gbs,
-                                         steps=min(args.steps, 10), warmup=3)
+                                         steps=args.steps, warmup=3)
 
     cpu = None
     if cpu_sample is not None:

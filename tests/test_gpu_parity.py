@@ -301,8 +301,8 @@ def test_float64_input_matches_float32_input(vet):
     e.close()
 
 
-def test_error_flags_map_to_reference_exceptions(vet):
-    cfg = vet.AnalyzerConfig(tile_counts=[20], output_dir=__import__("pathlib").Path("/tmp/vet_test_out"))
+def test_error_flags_map_to_reference_exceptions(vet, tmp_path):
+    cfg = vet.AnalyzerConfig(tile_counts=[20], output_dir=tmp_path)
     sa = vet.SpatialEntropyAnalyzer(cfg)
     ta = vet.TransitionEntropyAnalyzer(cfg)
     p = synth(3, 16, 1)
@@ -1051,14 +1051,14 @@ def test_naive_cell_table_every_cell_vs_reference(vet):
 
 
 @pytest.mark.parametrize("case", ["n_30_w", "n_30_u", "n_45x90_u", "n_10x20_w", "n_360_u", "n_3_u", "n_120x60_one"])
-def test_naive_frames_vs_reference_fixtures(vet, case):
+def test_naive_frames_vs_reference_fixtures(vet, case, tmp_path):
     """Packed path (streaming kernels with the grid table) and the functional API on RadialPoint dicts
     (k_naive_points) against compute_naive_spatial_entropy of the live reference; -inf / NaN quirks of
     a single 360x180 tile included."""
     c = _naive_golden()[f"frames/{case}"]
     tw, th = (int(x) for x in c["tile"])
     use_w = bool(c["use_w"])
-    cfg = vet.NaiveAnalyzerConfig(tile_width=tw, tile_height=th, output_dir=__import__("pathlib").Path("/tmp/vet_naive"),
+    cfg = vet.NaiveAnalyzerConfig(tile_width=tw, tile_height=th, output_dir=tmp_path,
                                   entropy_config=vet.EntropyConfig(use_weight_distribution=use_w))
     na = vet.NaiveSpatialEntropyAnalyzer(cfg)
     packed = c["packed"]

@@ -48,14 +48,14 @@ def test_library_exports_every_declared_symbol(pkg):
     assert b"FOV" in lib.vet_last_error()
 
 
-def test_no_cpu_fallback(pkg):
+def test_no_cpu_fallback(pkg, tmp_path):
     import torch
     if torch.cuda.is_available():
         pytest.skip("GPU present")
     with pytest.raises(RuntimeError, match="CUDA device"):
         pkg.Engine(100, 200, [20])
     with pytest.raises(RuntimeError, match="CUDA device"):
-        pkg.SpatialEntropyAnalyzer(pkg.AnalyzerConfig(output_dir=Path("/tmp/vet_t"))).engine
+        pkg.SpatialEntropyAnalyzer(pkg.AnalyzerConfig(output_dir=tmp_path)).engine
 
 
 def test_product_does_not_import_oracle():
@@ -237,6 +237,18 @@ def test_reference_named_ingest_functions(pkg, tmp_path):
                 assert v is None and p is None
             else:
                 assert (v.x, v.y, v.z) == tuple(vec[f, u]) and isinstance(p, pkg.RadialPoint)
+    # every point and vector against the reference's own decode chain, stored per pixel in the decode fixtures
+    # (lon / lat after the rounding and wrap of DU:390-397, Vector.from_spherical of every cell)
+    d = load_golden("decode")
+    px, py, _ = orc.decode(packed[..., 1], packed[..., 2], 100, 200)
+    checked = 0
+    for u, n in enumerate(names):
+        for f in np.flatnonzero(valid[:, u]):
+            v, p = vectors_df[n][f], points_df[n][f]
+            assert (p.lon, p.lat) == (d["lon_100x200"][px[f, u]], d["lat_100x200"][py[f, u]]), (n, f)
+            assert (v.x, v.y, v.z) == tuple(d["cellvec_100x200"][py[f, u], px[f, u]]), (n, f)
+            checked += 1
+    assert checked == int(valid.sum()) > 0
     with pytest.raises(pkg.ValidationError, match="Error processing viewport data"):
         pkg.process_viewport_data(tmp_path / "missing.csv", 100, 200)
     with pytest.raises(pkg.ValidationError, match="even numbers"):
