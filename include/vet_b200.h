@@ -251,6 +251,24 @@ int vet_analyze_host(vet_handle* h, const void* packed_host, int dtype, int64_t 
                      double* tr_entropy_host, double* tr_per_k_host, int32_t* prev_count0_host,
                      uint16_t* pairs0_host, int mode);
 
+/* Per-viewer exploration entropy: compute_spatial_entropy (EU:147-211) applied to the samples of ONE user over the
+ * frames of the video, averaged over the tile counts like SA:142-156 (semantics in vet_users.cuh).  A user without
+ * any present sample gets entropy NaN and a zero histogram row (the reference would raise "Empty vector
+ * dictionary"); frames without any present user are normal here (no VET_FLAG_EMPTY_FRAME).  Table regimes only:
+ * direct-only handles and the latitude/longitude grid tiling return VET_ERR_UNSUPPORTED.
+ *
+ * acc_dev: [U, S + 1] int64, S = sum_k T_k (tile counts concatenated in k order), column S = present samples.
+ * Adds this call's frames into acc (the caller zeroes it once); total_frames >= F fixes the fixed-point scale
+ * 2^-b, b = 62 - ceil(log2 total_frames) on weighted handles (0 on unweighted ones: plain counts).  The sums are
+ * exact integers, so frames added in any batching, order or over any number of ranks (acc summed across them)
+ * give the same bits when every call of one video passes the same total_frames (its global frame count). */
+int vet_users_accumulate(vet_handle* h, const void* packed_dev, int dtype, int64_t F, int64_t U,
+                         int64_t total_frames, int64_t* acc_dev, void* stream);
+/* acc -> entropy_dev[U], per_k_dev[K,U] (optional), hist0_dev[U,T_0] (optional, float64 tile weights of
+ * tile_counts[0]); total_frames as in the accumulating calls. */
+int vet_users_finish(vet_handle* h, const int64_t* acc_dev, int64_t U, int64_t total_frames,
+                     double* entropy_dev, double* per_k_dev, double* hist0_dev, void* stream);
+
 /* compute_naive_spatial_entropy (EU:362-453) for frames of ARBITRARY RadialPoints:
  * lonlat_dev[F,U,2] float64 degrees (NaN = absent user, EU:426-427) ->
  *   entropy_dev[F]     normalised entropy (NaN for a frame without users: the reference raises, flag word)

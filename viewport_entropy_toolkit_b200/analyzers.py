@@ -195,6 +195,34 @@ class SpatialEntropyAnalyzer(_AnalyzerBase):
             "tile_assignments": [LazyRowDict(assignments(f)) for f in range(F)]})
         return self._entropy_results
 
+    def compute_user_entropy(self, batch_bytes: int = 256 << 20) -> pd.DataFrame:
+        """Per-viewer exploration entropy: compute_spatial_entropy (EU:147-211) of each user's samples over the frames,
+        averaged over `config.tile_counts` -- how much of the sphere one viewer covered.  One row per user:
+        `identifier`, `frames` (frames with a sample), `entropy` (NaN for a user without any sample) and
+        `tile_weights`, a lazy {Vector: weight} dict of the user's summed tile weights of tile_counts[0].
+
+        The host array goes to the device in frame batches of about `batch_bytes` into one exact accumulator, so a
+        video larger than the GPU's memory works and the result does not depend on the batching."""
+        if not self._data_cache:
+            raise ValidationError("No data available. Call process_directory first.")
+        host = self._host_packed()
+        F, U = int(host.shape[0]), int(host.shape[1])
+        eng = self.engine
+        acc = eng.user_accumulator(U)
+        fb = max(1, int(batch_bytes) // max(1, U * 3 * host.itemsize))
+        for f0 in range(0, F, fb):
+            eng.users_accumulate(torch.from_numpy(host[f0:f0 + fb]).to(eng.device, non_blocking=True), acc, max(F, 1))
+        res = eng.users_finish(acc, max(F, 1), want_per_k=False)
+        eng.raise_for_flags()
+        ent, frames, hist0 = res.entropy.cpu().numpy(), res.frames.cpu().numpy(), res.hist0.cpu().numpy()
+        centres = self._fibonacci_vectors[self.config.tile_counts[0]]
+
+        def weights(u):
+            return lambda: {centres[i]: float(hist0[u, i]) for i in np.flatnonzero(hist0[u])}
+
+        return pd.DataFrame({"identifier": list(self._data_cache["identifiers"]), "frames": frames.astype(np.int64),
+                             "entropy": ent, "tile_weights": [LazyRowDict(weights(u)) for u in range(U)]})
+
 
 class TransitionEntropyAnalyzer(_AnalyzerBase):
     """Per-frame-pair transition entropy with the reference's literal bookkeeping

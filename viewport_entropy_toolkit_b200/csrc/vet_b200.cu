@@ -30,6 +30,7 @@
 #include "vet_whist.cuh"
 #include "vet_whist_i8.cuh"
 #include "vet_naive.cuh"
+#include "vet_users.cuh"
 
 #include "host/vet_host_core.inl"
 #include "host/vet_host_tables.inl"
@@ -39,3 +40,4 @@
 #include "host/vet_host_transition.inl"
 #include "host/vet_api_misc.inl"
 #include "host/vet_api_host.inl"
+#include "host/vet_host_users.inl"

@@ -9,6 +9,9 @@ order, EU:259-294).  The only collective is one all-gather of the packed per-fra
 rows [entropy | transition entropy | prev_count0]; tile assignments and the hist0
 rows stay sharded on the owning rank.
 
+`users_sharded` is the per-viewer counterpart: each rank adds its frames into an exact int64 per-user accumulator,
+one all_reduce(SUM) makes the rows complete on every rank.
+
 `analyze_sharded` is the product entry point (both analyzers, one pass over the
 rank's frames through Engine.analyze / vet_analyze); `run_sharded` is the generic
 wrapper around any per-rank compute function.
@@ -215,3 +218,39 @@ def analyze_sharded(engine, packed: Union[torch.Tensor, Callable[[int, int], tor
     sa = ShardedAnalyzer(engine, num_frames, group, rank, world, mode, want_hist0, want_assign0)
     local = packed(sa.read_begin, sa.end) if callable(packed) else packed
     return sa(local)
+
+
+def users_sharded(engine, packed: Union[torch.Tensor, Callable[[int, int], torch.Tensor]], num_frames: int,
+                  group=None, rank: Optional[int] = None, world: Optional[int] = None, want_per_k: bool = True,
+                  want_hist0: bool = True):
+    """Per-viewer exploration entropy (Engine.users) of a video of `num_frames` frames sharded by frames over the
+    ranks of `group`.  Every rank adds its own frame_range (no halo frame) into an int64 accumulator with the
+    fixed-point scale of the GLOBAL frame count, one all_reduce(SUM) adds the accumulators (integers: the order of
+    the ranks does not matter), and every rank finishes the complete rows: the UserResult is the same on every rank
+    and bit-identical to one GPU reading the whole video.  The collective moves U * (sum T_k + 1) * 8 bytes.
+
+    `packed` is this rank's frames [begin, end) of frame_range(num_frames, rank, world) as a device tensor, or a
+    callable load(frame_begin, frame_end) -> packed[frame_end - frame_begin, U, 3]."""
+    rank, world = _world(group, rank, world)
+    begin, end = frame_range(int(num_frames), rank, world)
+    local = packed(begin, end) if callable(packed) else packed
+    if local.dim() != 3 or local.shape[0] != end - begin:
+        raise ValueError(f"rank {rank} must be given frames [{begin}, {end}): {end - begin} frames, got {tuple(local.shape)}")
+    total = max(int(num_frames), 1)
+    acc = engine.user_accumulator(int(local.shape[1]))
+    if end > begin:
+        engine.users_accumulate(local, acc, total)
+    if world > 1:
+        all_reduce_accumulator(acc, group)
+    return engine.users_finish(acc, total, want_per_k, want_hist0)
+
+
+def all_reduce_accumulator(acc: torch.Tensor, group=None) -> None:
+    """Sums the int64 per-user accumulators of all ranks in place (one all_reduce); with the gloo backend a device
+    tensor is staged through host memory, as in all_gather_rows."""
+    if dist.get_backend(group) == "gloo" and acc.device.type == "cuda":
+        host = acc.cpu()
+        dist.all_reduce(host, op=dist.ReduceOp.SUM, group=group)
+        acc.copy_(host)
+    else:
+        dist.all_reduce(acc, op=dist.ReduceOp.SUM, group=group)

@@ -44,6 +44,15 @@ class TransitionResult:
     pairs0: Optional[torch.Tensor]       # [F-1, U, 2] uint16
 
 
+@dataclass
+class UserResult:
+    """Per-viewer exploration entropy: compute_spatial_entropy (EU:147-211) over one user's frames (vet_users_*)."""
+    entropy: torch.Tensor            # [U] float64, mean over tile counts; NaN for a user without any sample
+    per_k: Optional[torch.Tensor]    # [K, U] float64
+    hist0: Optional[torch.Tensor]    # [U, T0] float64 tile weights of tile_counts[0] summed over the user's frames
+    frames: torch.Tensor             # [U] int32 frames in which the user's sample is present
+
+
 def _check(rc: int) -> None:
     if rc == N.VET_OK:
         return
@@ -387,6 +396,63 @@ class Engine:
                                      _ptr(sp.assign0), tr.entropy.data_ptr(), _ptr(tr.per_k), _ptr(tr.prev_count0),
                                      _ptr(tr.pairs0), m, self._stream()))
         return sp, tr
+
+    # -- per-viewer exploration entropy ------------------------------------------------------
+    def user_accumulator(self, U: int) -> torch.Tensor:
+        """Zeroed int64 accumulator [U, sum(T_k) + 1] of users_accumulate (tile counts concatenated in k order, the last
+        column counts present samples)."""
+        return torch.zeros((int(U), sum(self.num_tiles) + 1), dtype=torch.int64, device=self.device)
+
+    def _check_acc(self, acc: torch.Tensor, U: Optional[int] = None) -> int:
+        if not isinstance(acc, torch.Tensor) or acc.device != self.device or acc.dtype != torch.int64:
+            raise TypeError("acc must be an int64 tensor on the engine's device (Engine.user_accumulator)")
+        if acc.dim() != 2 or acc.shape[1] != sum(self.num_tiles) + 1 or not acc.is_contiguous():
+            raise ValueError(f"acc must be a contiguous [U, {sum(self.num_tiles) + 1}] tensor")
+        if U is not None and acc.shape[0] != U:
+            raise ValueError(f"acc has {acc.shape[0]} user rows, packed has {U} users")
+        return int(acc.shape[0])
+
+    def users_accumulate(self, packed: torch.Tensor, acc: torch.Tensor, total_frames: int) -> None:
+        """Adds the frames of packed[F,U,3] into acc (vet_users_accumulate).  total_frames is the frame count of the
+        whole video: every batch (and every rank) of one video must pass the same value, which fixes the fixed-point
+        scale of the weights -- then any batching or frame order gives the same bits."""
+        p, dt = self._packed(packed)
+        if p.dim() != 3:
+            raise ValueError("packed must be [F, U, 3]")
+        F, U = int(p.shape[0]), int(p.shape[1])
+        self._check_acc(acc, U)
+        if int(total_frames) < max(F, 1):
+            raise ValueError(f"total_frames ({total_frames}) must be >= 1 and >= the frames of packed ({F})")
+        _check(self._lib.vet_users_accumulate(self._h, p.data_ptr(), dt, F, U, int(total_frames), acc.data_ptr(),
+                                              self._stream()))
+
+    def users_finish(self, acc: torch.Tensor, total_frames: int, want_per_k: bool = True,
+                     want_hist0: bool = True) -> UserResult:
+        """Entropies of finished accumulator rows (vet_users_finish); total_frames as in users_accumulate."""
+        U = self._check_acc(acc)
+        if int(total_frames) < 1:
+            raise ValueError("total_frames must be >= 1")
+        K, T0, dev = len(self.tile_counts), self.num_tiles[0], self.device
+        out = UserResult(
+            entropy=torch.empty(U, dtype=torch.float64, device=dev),
+            per_k=torch.empty((K, U), dtype=torch.float64, device=dev) if want_per_k else None,
+            hist0=torch.empty((U, T0), dtype=torch.float64, device=dev) if want_hist0 else None,
+            frames=acc[:, -1].to(torch.int32))
+        _check(self._lib.vet_users_finish(self._h, acc.data_ptr(), U, int(total_frames), out.entropy.data_ptr(),
+                                          _ptr(out.per_k), _ptr(out.hist0), self._stream()))
+        return out
+
+    def users(self, packed: torch.Tensor, want_per_k: bool = True, want_hist0: bool = True) -> UserResult:
+        """Per-viewer exploration entropy of packed[F,U,3]: compute_spatial_entropy (EU:147-211) of every user's
+        present samples over the frames, averaged over the tile counts (SA:142-156).  A user without any sample
+        gets NaN and a zero histogram row.  Call raise_for_flags() to raise for out-of-range coordinates."""
+        p, _ = self._packed(packed)
+        if p.dim() != 3:
+            raise ValueError("packed must be [F, U, 3]")
+        F, U = int(p.shape[0]), int(p.shape[1])
+        acc = self.user_accumulator(U)
+        self.users_accumulate(p, acc, max(F, 1))
+        return self.users_finish(acc, max(F, 1), want_per_k, want_hist0)
 
     # -- host-buffer (numpy) variants -----------------------------------------------------
     def spatial_host(self, packed: np.ndarray, want_per_k: bool = True, want_hist0: bool = True,
