@@ -114,9 +114,9 @@ enum {
   VET_OPT_STREAM_KERNEL = 1,     /* 0 auto, 1 plain loads (k_stream_simple), 2 cell histograms only (no direct tile
                                     histograms), 3 global-table regime without the 16-bit privatised histogram */
   VET_OPT_TRANSITION_KERNEL = 2, /* 0 auto (one-pass kernel k_transition4 where its tables fit, the two-pass kernels behind it),
-                                    1 k_transition, 2 k_transition2, 3 two-pass kernels (k_transition3 / 3c) */
-  VET_OPT_CLUSTER_TAIL = 3,      /* default 1: pairs left after the full rounds go to the cluster kernel when it pays;
-                                    0 never, 2 whenever it can run */
+                                    1 k_transition, 2 k_transition2, 3 two-pass kernel k_transition3 alone, one CTA per frame pair */
+  VET_OPT_CLUSTER_TAIL = 3,      /* default 1: the pairs the one-pass kernel has left after its full rounds go to its
+                                    cluster launch when it pays; 0 never, 2 whenever it can run */
   VET_OPT_T3_PAIR_SCRATCH = 4,   /* 1: keep the 4 B/user pair scratch also when the rows hold tile ids */
   VET_OPT_T3_ASSUME_MISSING = 5, /* 1: always test for missing users (no complete-frame variant) */
   VET_OPT_ANALYZE_OVERLAP = 6,   /* default 1: vet_analyze overlaps its spatial and transition stages; 0 runs them in sequence */
@@ -298,7 +298,8 @@ enum {
   VET_KERNEL_STREAM = 0,
   VET_KERNEL_EPILOGUE = 1,
   VET_KERNEL_TRANSITION = 2,
-  VET_KERNEL_TRANSITION_TAIL = 3, /* k_transition3c: the pairs left after the full rounds, one per CTA cluster */
+  VET_KERNEL_TRANSITION_TAIL = 3, /* k_transition4<true>: the pairs left after the full rounds, one per CTA cluster;
+                                     and k_transition3 over the pairs the one-pass kernel flags */
   VET_KERNEL_COUNT = 4
 };
 int vet_profile_enable(vet_handle* h, int on);

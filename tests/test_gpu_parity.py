@@ -873,44 +873,48 @@ def test_transition_two_pass_kernel_equals_three_pass_kernel(vet, U):
 
 @pytest.mark.parametrize("F,U,tcs", [
     (3, 66_000, [200]),          # 2 pairs, clusters of 8, tile ids straight from the streaming kernel
-    (3, 40_001, [200, 20]),      # clusters of 4, odd U (scalar loads), LUTs staged in shared memory
-    (152, 16_384, [200]),        # 151 pairs: one full round of k_transition3 + 3 pairs on clusters of 2
+    (3, 40_001, [200, 20]),      # clusters of 4, odd U (scalar loads), rows relabelled to tile ids
+    (152, 16_384, [200]),        # 151 pairs: one full round of k_transition4 + 3 pairs on clusters of 2
     (21, 131_072, [100, 200]),   # 20 pairs: more than the co-resident clusters of 8
 ])
-def test_transition_cluster_tail_equals_single_cta(vet, F, U, tcs):
-    """k_transition3c (the users of one frame pair split over a thread-block cluster, for the pairs left after
-    the full rounds) against k_transition3 alone: every output bit for bit, transition() and analyze();
-    the small cases also against the oracle."""
+def test_one_pass_cluster_tail_equals_single_cta(vet, F, U, tcs):
+    """k_transition4<true> (the users of one frame pair split over a thread-block cluster, for the pairs left after
+    the full rounds) against the one-pass kernel without it and against k_transition3 alone: every output bit for bit,
+    transition() and analyze(); the small cases also against the oracle."""
     import bench
     p = bench.synth_on_device(torch, F, U, 616 + U, torch.device("cuda"))
     p[1, ::5, 1] = float("nan")                                   # missing users
     g = torch.Generator(device="cuda").manual_seed(7)
     p[F - 2:, :, 1:] = torch.rand((2, U, 2), generator=g, device="cuda")   # iid frames: every row of the table in use
     e = engine(vet, tcs, use_w=False)
-    e.set_option("transition_kernel", "v3")   # the two-pass kernels themselves (auto puts the one-pass kernel in front)
     res = {}
     e.profile(True)
-    for cl in ("0", "force"):      # force: also below the frame size from which the host picks it by itself
-        e.set_option("cluster_tail", "off" if cl == "0" else "force")
+    # force: also below the frame size from which the host picks the clusters by itself; v3: one CTA per pair
+    for name, tk, cl in (("v3", "v3", "off"), ("0", "auto", "off"), ("force", "auto", "force")):
+        e.set_option("transition_kernel", tk)
+        e.set_option("cluster_tail", cl)
         tr = e.transition(p)
         _, tr2 = e.analyze(p)
         assert e.poll_flags() == 0
-        res[cl] = (tr, tr2, e.profile_read()["transition_tail"][1])
+        res[name] = (tr, tr2, e.profile_read()["transition_tail"][1])
     e.profile(False)
-    assert res["0"][2] == 0 and res["force"][2] == 2 * len(tcs), "one cluster launch per tile count and call"
+    # transition_tail also counts the k_transition3 pass over the pairs k_transition4 flags, once per tile count and call
+    assert res["v3"][2] == 0 and res["force"][2] - res["0"][2] == 2 * len(tcs), "one cluster launch per tile count and call"
     # the same without the shortcuts of k_transition3: missing-user tests kept for complete frames, pair scratch kept
+    e.set_option("transition_kernel", "v3")
     e.set_option("cluster_tail", "off")
     e.set_option("t3_assume_missing", "on")
     e.set_option("t3_pair_scratch", "on")
     plain = e.transition(p)
     e.set_option("t3_assume_missing", "off")
     e.set_option("t3_pair_scratch", "off")
-    assert torch.equal(plain.pairs0, res["0"][0].pairs0) and torch.equal(plain.prev_count0, res["0"][0].prev_count0)
-    assert np.array_equal(plain.entropy.cpu().numpy(), res["0"][0].entropy.cpu().numpy(), equal_nan=True)
-    for a, b in ((res["0"][0], res["force"][0]), (res["0"][0], res["force"][1])):
-        assert torch.equal(a.pairs0, b.pairs0) and torch.equal(a.prev_count0, b.prev_count0)
-        assert np.array_equal(a.per_k.cpu().numpy(), b.per_k.cpu().numpy(), equal_nan=True)
-        assert np.array_equal(a.entropy.cpu().numpy(), b.entropy.cpu().numpy(), equal_nan=True)
+    assert torch.equal(plain.pairs0, res["v3"][0].pairs0) and torch.equal(plain.prev_count0, res["v3"][0].prev_count0)
+    assert np.array_equal(plain.entropy.cpu().numpy(), res["v3"][0].entropy.cpu().numpy(), equal_nan=True)
+    for name in ("0", "force"):
+        for a, b in ((res["v3"][0], res[name][0]), (res["v3"][0], res[name][1])):
+            assert torch.equal(a.pairs0, b.pairs0) and torch.equal(a.prev_count0, b.prev_count0), name
+            assert np.array_equal(a.per_k.cpu().numpy(), b.per_k.cpu().numpy(), equal_nan=True), name
+            assert np.array_equal(a.entropy.cpu().numpy(), b.entropy.cpu().numpy(), equal_nan=True), name
     if F <= 3:
         ref = orc.transition_analyzer(p.cpu().numpy(), W0, H0, tcs, mode="literal")
         b = res["force"][0]

@@ -25,11 +25,9 @@ walk[1:, :, 1:] = (walk[:1, :, 1:] + 0.004 * torch.arange(1, 4, device="cuda")[:
 tw = e.transition(walk)                             # k_transition4 on its tables (ranked tile deltas), list of a few users
 e.set_option("cluster_tail", "force")
 twc = e.transition(walk)                            # k_transition4<cluster>: tables merged into CTA 0 through DSMEM atomics
-e.set_option("transition_kernel", "v3")
-tc = e.transition(packed(3, 16384))                 # k_transition3c: a frame pair per cluster of 2 CTAs (tables merged through DSMEM)
+tc = e.transition(packed(3, 16384))                 # k_transition4<cluster>: a frame pair per cluster of 2 CTAs, iid samples
 sa, ta = e.analyze(packed(3, 16384))                # the same with the spatial epilogue on the side stream beside it
 e.set_option("cluster_tail", "auto")
-e.set_option("transition_kernel", "auto")
 e.set_option("weighted_kernel", "i8")
 hot = packed(140, 2504)
 hot[:, :600, 1:] = 0.5                              # 600 users in one cell: second count plane

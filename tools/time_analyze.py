@@ -29,8 +29,8 @@ def timed(fn, n=5):
     return a.elapsed_time(b) / n
 
 
-for tk, overlap, cl in (("auto", "on", "auto"), ("v3", "on", "auto"), ("v3", "off", "auto")):
-    eng.set_option("transition_kernel", tk)   # auto: fused streaming + transition pass; v3: two-pass kernels behind the stream
+for tk, overlap, cl in (("auto", "on", "auto"), ("auto", "on", "off"), ("v3", "on", "off"), ("v3", "off", "off")):
+    eng.set_option("transition_kernel", tk)   # auto: one-pass kernel (cluster_tail: its clusters for the last pairs); v3: two-pass kernel alone
     eng.set_option("analyze_overlap", overlap)
     eng.set_option("cluster_tail", cl)
     eng.profile(True)

@@ -24,7 +24,6 @@
 #include "vet_transition.cuh"
 #include "vet_transition2.cuh"
 #include "vet_transition3.cuh"
-#include "vet_transition3c.cuh"
 #include "vet_transition4.cuh"
 #include "vet_vectors.cuh"
 #include "vet_whist.cuh"

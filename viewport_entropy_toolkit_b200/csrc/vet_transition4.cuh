@@ -68,7 +68,7 @@ __device__ __forceinline__ void t4_inc(uint32_t addr) {
   asm volatile("red.shared.add.u32 [%0], 1;" ::"r"(addr) : "memory");
 }
 
-// CL: one frame pair per thread-block CLUSTER (the pairs left after the full rounds, like k_transition3c): the CTAs of
+// CL: one frame pair per thread-block CLUSTER (the pairs left after the full rounds of one pair per SM): the CTAs of
 // a cluster take interleaved steps of the users into their own tables, then push their non-empty entries into the
 // tables of CTA 0 through distributed shared memory (add / two-level min -- the same integers as one CTA would
 // have collected), and CTA 0 finishes the pair.
