@@ -269,6 +269,25 @@ int vet_users_accumulate(vet_handle* h, const void* packed_dev, int dtype, int64
 int vet_users_finish(vet_handle* h, const int64_t* acc_dev, int64_t U, int64_t total_frames,
                      double* entropy_dev, double* per_k_dev, double* hist0_dev, void* stream);
 
+/* Tile transition matrix of a video (semantics in vet_transition_counts.cuh): n_k[p, c] = the (frame pair (f, f+1),
+ * user) combinations with the user present in both frames, on tile p of tile count k in frame f and on tile c in
+ * frame f+1 -- the pairs of EU:271-276, unweighted -- summed over the frame pairs of the call, and the pooled
+ * conditional entropy H_k = -sum (n_pc / N) log2(n_pc / n_p), normalised like the textbook mode (EU:321-327), mean over
+ * k.  N = 0, N = 1 and T = 1 give NaN.  A frame pair without a common user raises no flag; out-of-range coordinates set
+ * VET_FLAG_OUT_OF_RANGE and count as missing.  Table regimes only: direct-only handles, the latitude/longitude grid
+ * tiling and sum_k T_k^2 > 2^28 return VET_ERR_UNSUPPORTED.  Neither call synchronises the stream.
+ *
+ * acc_dev: int64, the [T_k, T_k] count matrices of all tile counts concatenated in k order (row = previous tile).
+ * Adds the (f, f+1) pairs of packed_dev[F,U,3] into acc (the caller zeroes it once).  Batches that overlap by one frame
+ * add up to the whole video; the sums are exact integers, so any batching or sharding gives the same bits. */
+int vet_transition_counts_accumulate(vet_handle* h, const void* packed_dev, int dtype, int64_t F, int64_t U,
+                                     int64_t* acc_dev, void* stream);
+/* acc -> entropy_dev[1] (mean over k), per_k_dev[K] (optional), pairs_dev[1] (optional, int64 N).  The row sums go
+ * through scratch the handle allocates at creation: finish calls of one handle on different streams must be ordered,
+ * like every other call that uses the handle's scratch. */
+int vet_transition_counts_finish(vet_handle* h, const int64_t* acc_dev, double* entropy_dev, double* per_k_dev,
+                                 int64_t* pairs_dev, void* stream);
+
 /* compute_naive_spatial_entropy (EU:362-453) for frames of ARBITRARY RadialPoints:
  * lonlat_dev[F,U,2] float64 degrees (NaN = absent user, EU:426-427) ->
  *   entropy_dev[F]     normalised entropy (NaN for a frame without users: the reference raises, flag word)

@@ -47,6 +47,8 @@ r2 = e.spatial(packed(9, 3001, np.float64))         # k_stream_tiles (direct unw
 r3 = e.spatial(packed(3, 90001))                    # cells path: k_stream_tma + k_epilogue, several chunks per frame
 t2 = e.transition(packed(3, 20000))                 # k_transition3 hash, overflow -> rows redone by k_transition2 (global tables)
 t3 = e.transition(packed(5, 700), mode="textbook")  # k_transition (shared-memory table)
+tcn = e.transition_counts(packed(6, 3001))          # k_tc_count (ranked deltas for 21/51 tiles, global atomics for 1001) +
+                                                    # k_tc_rows + k_tc_entropy
 e.close()
 e = Engine(200, 400, [20], EntropyConfig())
 r4 = e.spatial(packed(2, 300))                      # global-table regime, weighted: k_stream_frame16 + k_whist

@@ -93,6 +93,8 @@ SYMBOLS = {
     "vet_analyze_host": (C.c_int, [_P, _P, C.c_int, _I64, _I64, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int]),
     "vet_users_accumulate": (C.c_int, [_P, _P, C.c_int, _I64, _I64, _I64, _P, _P]),
     "vet_users_finish": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _P, _P]),
+    "vet_transition_counts_accumulate": (C.c_int, [_P, _P, C.c_int, _I64, _I64, _P, _P]),
+    "vet_transition_counts_finish": (C.c_int, [_P, _P, _P, _P, _P, _P]),
     "vet_naive_points": (C.c_int, [_P, _P, _I64, _I64, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     "vet_poll_flags": (C.c_int, [_P, _P, C.POINTER(C.c_uint32)]),
     "vet_launch_count": (_I64, [_P]),

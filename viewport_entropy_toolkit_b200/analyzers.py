@@ -262,6 +262,25 @@ class TransitionEntropyAnalyzer(_AnalyzerBase):
             "tile_assignments": [LazyRowDict(assignments(r)) for r in range(R)]})
         return self._entropy_results
 
+    def compute_transition_counts(self, batch_bytes: int = 256 << 20) -> Dict:
+        """Tile transition matrix of the video: per tile count of `config.tile_counts` the [T, T] int64 numpy array
+        of users moving from tile p in one frame to tile c in the next, summed over all frame pairs, and the pooled
+        conditional entropy.  Returns dict(counts=[...], entropy=float, per_k=[K] float64, pairs=int).
+
+        The host array goes to the device in frame batches of about `batch_bytes` that overlap by one frame, into one
+        exact accumulator: a video larger than the GPU's memory works and the result does not depend on the batching."""
+        host = self._host_packed()
+        F, U = int(host.shape[0]), int(host.shape[1])
+        eng = self.engine
+        acc = eng.transition_counts_accumulator()
+        fb = max(2, int(batch_bytes) // max(1, U * 3 * host.itemsize))
+        for f0 in range(0, max(F - 1, 1), fb - 1):
+            eng.transition_counts_accumulate(torch.from_numpy(host[f0:f0 + fb]).to(eng.device, non_blocking=True), acc)
+        res = eng.transition_counts_finish(acc)
+        eng.raise_for_flags()
+        return dict(counts=[c.cpu().numpy() for c in res.counts], entropy=float(res.entropy),
+                    per_k=res.per_k.cpu().numpy(), pairs=res.pairs)
+
 
 class NaiveSpatialEntropyAnalyzer(_AnalyzerBase):
     """Per-frame normalised Shannon entropy over a latitude/longitude grid of tile_width x

@@ -30,6 +30,7 @@
 #include "vet_whist_i8.cuh"
 #include "vet_naive.cuh"
 #include "vet_users.cuh"
+#include "vet_transition_counts.cuh"
 
 #include "host/vet_host_core.inl"
 #include "host/vet_host_tables.inl"
@@ -40,3 +41,4 @@
 #include "host/vet_api_misc.inl"
 #include "host/vet_api_host.inl"
 #include "host/vet_host_users.inl"
+#include "host/vet_host_transition_counts.inl"

@@ -10,7 +10,8 @@ rows [entropy | transition entropy | prev_count0]; tile assignments and the hist
 rows stay sharded on the owning rank.
 
 `users_sharded` is the per-viewer counterpart: each rank adds its frames into an exact int64 per-user accumulator,
-one all_reduce(SUM) makes the rows complete on every rank.
+one all_reduce(SUM) makes the rows complete on every rank.  `transition_counts_sharded` does the same for the tile
+transition matrix, each rank reading its frames plus the halo frame.
 
 `analyze_sharded` is the product entry point (both analyzers, one pass over the
 rank's frames through Engine.analyze / vet_analyze); `run_sharded` is the generic
@@ -245,8 +246,32 @@ def users_sharded(engine, packed: Union[torch.Tensor, Callable[[int, int], torch
     return engine.users_finish(acc, total, want_per_k, want_hist0)
 
 
+def transition_counts_sharded(engine, packed: Union[torch.Tensor, Callable[[int, int], torch.Tensor]], num_frames: int,
+                              group=None, rank: Optional[int] = None, world: Optional[int] = None):
+    """Tile transition matrix (Engine.transition_counts) of a video of `num_frames` frames sharded by frames over the
+    ranks of `group`.  Every rank reads [read_begin, end) of analyze_read_range -- its own frames plus the halo frame --
+    and counts the frame pairs inside it, so each pair is counted by exactly one rank; one all_reduce(SUM) of the
+    sum_k T_k^2 int64 counts adds the ranks (integers: order-free), and every rank finishes locally: the
+    TransitionCountsResult is the same on every rank and bit-identical to one GPU reading the whole video.
+
+    `packed` is this rank's frames [read_begin, end) as a device tensor, or a callable
+    load(frame_begin, frame_end) -> packed[frame_end - frame_begin, U, 3]."""
+    rank, world = _world(group, rank, world)
+    read_begin, _, end = analyze_read_range(int(num_frames), rank, world)
+    local = packed(read_begin, end) if callable(packed) else packed
+    if local.dim() != 3 or local.shape[0] != end - read_begin:
+        raise ValueError(f"rank {rank} must be given frames [{read_begin}, {end}): {end - read_begin} frames, "
+                         f"got {tuple(local.shape)}")
+    acc = engine.transition_counts_accumulator()
+    if end > read_begin:
+        engine.transition_counts_accumulate(local, acc)
+    if world > 1:
+        all_reduce_accumulator(acc, group)
+    return engine.transition_counts_finish(acc)
+
+
 def all_reduce_accumulator(acc: torch.Tensor, group=None) -> None:
-    """Sums the int64 per-user accumulators of all ranks in place (one all_reduce); with the gloo backend a device
+    """Sums the int64 accumulators (per-user rows, transition counts) of all ranks in place (one all_reduce); with the gloo backend a device
     tensor is staged through host memory, as in all_gather_rows."""
     if dist.get_backend(group) == "gloo" and acc.device.type == "cuda":
         host = acc.cpu()

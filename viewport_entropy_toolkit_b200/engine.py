@@ -53,6 +53,16 @@ class UserResult:
     frames: torch.Tensor             # [U] int32 frames in which the user's sample is present
 
 
+@dataclass
+class TransitionCountsResult:
+    """Tile transition matrix of a video (vet_transition_counts_*): counts[k][p, c] = (frame pair, user) combinations
+    moving from tile p to tile c of tile count k, and their pooled conditional entropy."""
+    counts: List[torch.Tensor]       # per tile count a [T_k, T_k] int64 view of the accumulator (row = previous tile)
+    entropy: torch.Tensor            # 0-d float64, mean over tile counts; NaN without any pair
+    per_k: torch.Tensor              # [K] float64
+    pairs: int                       # N: (frame pair, user) combinations with the user present in both frames
+
+
 def _check(rc: int) -> None:
     if rc == N.VET_OK:
         return
@@ -453,6 +463,53 @@ class Engine:
         acc = self.user_accumulator(U)
         self.users_accumulate(p, acc, max(F, 1))
         return self.users_finish(acc, max(F, 1), want_per_k, want_hist0)
+
+    # -- tile transition matrix ----------------------------------------------------------------
+    def transition_counts_accumulator(self) -> torch.Tensor:
+        """Zeroed int64 accumulator of transition_counts_accumulate: the [T_k, T_k] matrices of all tile counts,
+        flattened and concatenated in k order."""
+        return torch.zeros(sum(t * t for t in self.num_tiles), dtype=torch.int64, device=self.device)
+
+    def _check_tc_acc(self, acc: torch.Tensor) -> None:
+        n = sum(t * t for t in self.num_tiles)
+        if not isinstance(acc, torch.Tensor) or acc.device != self.device or acc.dtype != torch.int64:
+            raise TypeError("acc must be an int64 tensor on the engine's device (Engine.transition_counts_accumulator)")
+        if acc.dim() != 1 or acc.shape[0] != n or not acc.is_contiguous():
+            raise ValueError(f"acc must be a contiguous [{n}] tensor")
+
+    def transition_counts_accumulate(self, packed: torch.Tensor, acc: torch.Tensor) -> None:
+        """Adds the (f, f+1) frame pairs of packed[F,U,3] into acc (vet_transition_counts_accumulate).  Batches that
+        overlap by one frame add up to the whole video, in any batching and order, with the same bits."""
+        p, dt = self._packed(packed)
+        if p.dim() != 3:
+            raise ValueError("packed must be [F, U, 3]")
+        self._check_tc_acc(acc)
+        _check(self._lib.vet_transition_counts_accumulate(self._h, p.data_ptr(), dt, int(p.shape[0]), int(p.shape[1]),
+                                                          acc.data_ptr(), self._stream()))
+
+    def transition_counts_finish(self, acc: torch.Tensor) -> TransitionCountsResult:
+        """Pooled conditional entropy of the finished counts (vet_transition_counts_finish); `counts` are views of acc.
+        Synchronises the current stream to read the pair count."""
+        self._check_tc_acc(acc)
+        K, dev = len(self.tile_counts), self.device
+        entropy = torch.empty((), dtype=torch.float64, device=dev)
+        per_k = torch.empty(K, dtype=torch.float64, device=dev)
+        pairs = torch.empty(1, dtype=torch.int64, device=dev)
+        _check(self._lib.vet_transition_counts_finish(self._h, acc.data_ptr(), entropy.data_ptr(), per_k.data_ptr(),
+                                                      pairs.data_ptr(), self._stream()))
+        counts, off = [], 0
+        for t in self.num_tiles:
+            counts.append(acc[off:off + t * t].view(t, t))
+            off += t * t
+        return TransitionCountsResult(counts=counts, entropy=entropy, per_k=per_k, pairs=int(pairs.item()))
+
+    def transition_counts(self, packed: torch.Tensor) -> TransitionCountsResult:
+        """Tile transition matrix of packed[F,U,3]: per tile count the users moving from tile p in frame f to tile c in
+        frame f+1, summed over all frame pairs, and the pooled conditional entropy -sum (n_pc/N) log2(n_pc/n_p)
+        normalised like the textbook mode.  Call raise_for_flags() to raise for out-of-range coordinates."""
+        acc = self.transition_counts_accumulator()
+        self.transition_counts_accumulate(packed, acc)
+        return self.transition_counts_finish(acc)
 
     # -- host-buffer (numpy) variants -----------------------------------------------------
     def spatial_host(self, packed: np.ndarray, want_per_k: bool = True, want_hist0: bool = True,
