@@ -288,6 +288,22 @@ int vet_transition_counts_accumulate(vet_handle* h, const void* packed_dev, int 
 int vet_transition_counts_finish(vet_handle* h, const int64_t* acc_dev, double* entropy_dev, double* per_k_dev,
                                  int64_t* pairs_dev, void* stream);
 
+/* Per-viewer transition entropy (semantics in vet_user_transitions.cuh): for every user u the conditional entropy of
+ * the next tile given the current one over u's own frames -- transition_entropy_textbook (EU:321-327 normalisation) of
+ * the (prev_idx, cur_idx) pairs (EU:271-276) of the frames f where u is present in f and f+1, unweighted -- per tile
+ * count, and its sequential mean over k (SA:151-156).  One deliberate deviation: a user without a pair (N_u = 0) gets
+ * NaN where the textbook mode would raise ZeroDivisionError; N_u = 1 and T = 1 give NaN as in the textbook mode.
+ * Out-of-range coordinates set VET_FLAG_OUT_OF_RANGE and count as missing.  A user's outputs are the same bits
+ * whatever other users share the call, in any user order, batching or sharding.  Table regimes only: direct-only
+ * handles and the latitude/longitude grid tiling return VET_ERR_UNSUPPORTED, and so does F - 1 >= 2^31.  U = 0 or
+ * F < 2 is a valid call (every user NaN, 0 pairs).
+ *
+ * entropy_dev[U]; per_k_dev[K,U] optional; pairs_dev[U] int32 (N_u) optional.  One call = every frame of these U
+ * users.  Does not synchronise; after the first call of a size it does not allocate (scratch grown with the handle). */
+#define VET_UT_SMEM_RECORDS 3712  /* pair records (runs of one repeated pair) a user's sort keeps in shared memory */
+int vet_user_transitions(vet_handle* h, const void* packed_dev, int dtype, int64_t F, int64_t U,
+                         double* entropy_dev, double* per_k_dev, int32_t* pairs_dev, void* stream);
+
 /* compute_naive_spatial_entropy (EU:362-453) for frames of ARBITRARY RadialPoints:
  * lonlat_dev[F,U,2] float64 degrees (NaN = absent user, EU:426-427) ->
  *   entropy_dev[F]     normalised entropy (NaN for a frame without users: the reference raises, flag word)
@@ -309,7 +325,7 @@ int64_t vet_launch_count(const vet_handle* h);
 int64_t vet_graph_replays(const vet_handle* h);
 
 /* Per-kernel device timing for the benchmark's roofline line.  When enabled, every
- * launch of the streaming / epilogue / transition / transition-tail kernels is bracketed by a CUDA
+ * launch of the streaming / epilogue / transition / transition-tail / per-viewer transition kernels is bracketed by a CUDA
  * event pair on its own stream (no synchronisation is added).  vet_profile_read
  * waits for the recorded events, returns the summed milliseconds and launch counts
  * per kernel (arrays of VET_KERNEL_COUNT) and clears the record. */
@@ -319,7 +335,9 @@ enum {
   VET_KERNEL_TRANSITION = 2,
   VET_KERNEL_TRANSITION_TAIL = 3, /* k_transition4<true>: the pairs left after the full rounds, one per CTA cluster;
                                      and k_transition3 over the pairs the one-pass kernel flags */
-  VET_KERNEL_COUNT = 4
+  VET_KERNEL_USER_ROWS = 4,       /* k_ut_rows of vet_user_transitions */
+  VET_KERNEL_USER_ENTROPY = 5,    /* k_ut_entropy of vet_user_transitions */
+  VET_KERNEL_COUNT = 6
 };
 int vet_profile_enable(vet_handle* h, int on);
 int vet_profile_read(vet_handle* h, double* ms_by_kernel, int64_t* launches_by_kernel);

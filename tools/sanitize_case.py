@@ -49,6 +49,7 @@ t2 = e.transition(packed(3, 20000))                 # k_transition3 hash, overfl
 t3 = e.transition(packed(5, 700), mode="textbook")  # k_transition (shared-memory table)
 tcn = e.transition_counts(packed(6, 3001))          # k_tc_count (ranked deltas for 21/51 tiles, global atomics for 1001) +
                                                     # k_tc_rows + k_tc_entropy
+ut = e.user_transitions(packed(3801, 7))            # k_ut_rows + k_ut_entropy (records past shared memory: global slices)
 e.close()
 e = Engine(200, 400, [20], EntropyConfig())
 r4 = e.spatial(packed(2, 300))                      # global-table regime, weighted: k_stream_frame16 + k_whist

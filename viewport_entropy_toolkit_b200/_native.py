@@ -27,6 +27,9 @@ VET_REGIME_AUTO, VET_REGIME_DIRECT = 0, 1
 # include/vet_b200.h VET_I8_MIN_FRAMES: frames per call from which the automatic dispatch of the weighted histogram
 # takes the tensor-core kernel (tests/test_host_logic.py checks the two against each other)
 I8_MIN_FRAMES = 384
+# include/vet_b200.h VET_UT_SMEM_RECORDS: pair records of one user that vet_user_transitions sorts in shared memory;
+# more go through global scratch (the tests cover both sides)
+UT_SMEM_RECORDS = 3712
 
 OPTIONS = {
     "weighted_kernel": (0, {"auto": 0, "fp64": 1, "i8": 2}),
@@ -95,6 +98,7 @@ SYMBOLS = {
     "vet_users_finish": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _P, _P]),
     "vet_transition_counts_accumulate": (C.c_int, [_P, _P, C.c_int, _I64, _I64, _P, _P]),
     "vet_transition_counts_finish": (C.c_int, [_P, _P, _P, _P, _P, _P]),
+    "vet_user_transitions": (C.c_int, [_P, _P, C.c_int, _I64, _I64, _P, _P, _P, _P]),
     "vet_naive_points": (C.c_int, [_P, _P, _I64, _I64, C.c_int32, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     "vet_poll_flags": (C.c_int, [_P, _P, C.POINTER(C.c_uint32)]),
     "vet_launch_count": (_I64, [_P]),
@@ -102,7 +106,7 @@ SYMBOLS = {
     "vet_profile_enable": (C.c_int, [_P, C.c_int]),
     "vet_profile_read": (C.c_int, [_P, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
 }
-KERNEL_NAMES = ("stream", "epilogue", "transition", "transition_tail")  # VET_KERNEL_* of vet_b200.h
+KERNEL_NAMES = ("stream", "epilogue", "transition", "transition_tail", "user_rows", "user_entropy")  # VET_KERNEL_* of vet_b200.h
 
 _lib: Optional[C.CDLL] = None
 

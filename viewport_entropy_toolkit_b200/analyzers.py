@@ -281,6 +281,28 @@ class TransitionEntropyAnalyzer(_AnalyzerBase):
         return dict(counts=[c.cpu().numpy() for c in res.counts], entropy=float(res.entropy),
                     per_k=res.per_k.cpu().numpy(), pairs=res.pairs)
 
+    def compute_user_transition_entropy(self, batch_bytes: int = 256 << 20) -> pd.DataFrame:
+        """Per-viewer transition entropy: the textbook conditional entropy (EU:321-327) of each user's own moves from
+        tile p in one frame to tile c in the next, averaged over `config.tile_counts` -- how predictable one viewer's
+        movement is.  One row per user: `identifier`, `pairs` (frames f with the user present in f and f+1) and
+        `entropy` (NaN for a user without any pair).
+
+        A user's result depends on that user's samples only, so the host array goes to the device in blocks of user
+        columns (all frames of about `batch_bytes` worth of users): a video larger than the GPU's memory works and the
+        result does not depend on the batching."""
+        host = self._host_packed()
+        F, U = int(host.shape[0]), int(host.shape[1])
+        eng = self.engine
+        ub = max(1, int(batch_bytes) // max(1, F * 3 * host.itemsize))
+        ent, pairs = np.empty(U, dtype=np.float64), np.empty(U, dtype=np.int64)
+        for u0 in range(0, U, ub):
+            block = torch.from_numpy(np.ascontiguousarray(host[:, u0:u0 + ub])).to(eng.device, non_blocking=True)
+            res = eng.user_transitions(block, want_per_k=False)
+            ent[u0:u0 + ub] = res.entropy.cpu().numpy()
+            pairs[u0:u0 + ub] = res.pairs.cpu().numpy()
+        eng.raise_for_flags()
+        return pd.DataFrame({"identifier": list(self._data_cache["identifiers"]), "pairs": pairs, "entropy": ent})
+
 
 class NaiveSpatialEntropyAnalyzer(_AnalyzerBase):
     """Per-frame normalised Shannon entropy over a latitude/longitude grid of tile_width x

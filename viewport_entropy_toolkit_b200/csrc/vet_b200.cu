@@ -31,6 +31,7 @@
 #include "vet_naive.cuh"
 #include "vet_users.cuh"
 #include "vet_transition_counts.cuh"
+#include "vet_user_transitions.cuh"
 
 #include "host/vet_host_core.inl"
 #include "host/vet_host_tables.inl"
@@ -42,3 +43,4 @@
 #include "host/vet_api_host.inl"
 #include "host/vet_host_users.inl"
 #include "host/vet_host_transition_counts.inl"
+#include "host/vet_host_user_transitions.inl"

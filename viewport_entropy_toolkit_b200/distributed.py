@@ -11,7 +11,9 @@ rows stay sharded on the owning rank.
 
 `users_sharded` is the per-viewer counterpart: each rank adds its frames into an exact int64 per-user accumulator,
 one all_reduce(SUM) makes the rows complete on every rank.  `transition_counts_sharded` does the same for the tile
-transition matrix, each rank reading its frames plus the halo frame.
+transition matrix, each rank reading its frames plus the halo frame.  `user_transitions_sharded` shards by users
+instead: a viewer's transition entropy needs all of that viewer's frames and nothing of the other viewers, so each rank
+reads the columns of its users and one all-gather of the per-user rows completes the result.
 
 `analyze_sharded` is the product entry point (both analyzers, one pass over the
 rank's frames through Engine.analyze / vet_analyze); `run_sharded` is the generic
@@ -26,6 +28,7 @@ import torch
 import torch.distributed as dist
 
 from . import _native
+from .engine import UserTransitionResult
 
 
 def frame_range(num_frames: int, rank: int, world: int) -> Tuple[int, int]:
@@ -268,6 +271,30 @@ def transition_counts_sharded(engine, packed: Union[torch.Tensor, Callable[[int,
     if world > 1:
         all_reduce_accumulator(acc, group)
     return engine.transition_counts_finish(acc)
+
+
+def user_transitions_sharded(engine, packed: Union[torch.Tensor, Callable[[int, int], torch.Tensor]], num_users: int,
+                             group=None, rank: Optional[int] = None, world: Optional[int] = None,
+                             want_per_k: bool = True):
+    """Per-viewer transition entropy (Engine.user_transitions) of a video of `num_users` users sharded by USERS over
+    the ranks of `group`: a user's result depends on that user's samples only, over all frames, so rank r owns the
+    users frame_range(num_users, r, world) and computes them from their columns alone.  One all_gather_rows of the
+    per-user rows [entropy | pairs | per_k] makes the UserTransitionResult complete on every rank, bit-identical to one
+    GPU reading the whole video.
+
+    `packed` is this rank's user columns [F, u1 - u0, 3] as a device tensor, or a callable
+    load(user_begin, user_end) -> packed[F, user_end - user_begin, 3]."""
+    rank, world = _world(group, rank, world)
+    u0, u1 = frame_range(int(num_users), rank, world)
+    local = packed(u0, u1) if callable(packed) else packed
+    if local.dim() != 3 or local.shape[1] != u1 - u0:
+        raise ValueError(f"rank {rank} must be given users [{u0}, {u1}): {u1 - u0} users, got {tuple(local.shape)}")
+    res = engine.user_transitions(local, want_per_k)
+    cols = [res.entropy[:, None], res.pairs.to(torch.float64)[:, None]] + ([res.per_k.t()] if want_per_k else [])
+    counts = [frame_range(int(num_users), r, world)[1] - frame_range(int(num_users), r, world)[0] for r in range(world)]
+    full = all_gather_rows(torch.cat(cols, 1), counts, group)
+    return UserTransitionResult(entropy=full[:, 0].contiguous(), per_k=full[:, 2:].t().contiguous() if want_per_k else None,
+                                pairs=full[:, 1].to(torch.int32))
 
 
 def all_reduce_accumulator(acc: torch.Tensor, group=None) -> None:

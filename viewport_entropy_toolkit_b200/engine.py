@@ -63,6 +63,15 @@ class TransitionCountsResult:
     pairs: int                       # N: (frame pair, user) combinations with the user present in both frames
 
 
+@dataclass
+class UserTransitionResult:
+    """Per-viewer transition entropy (vet_user_transitions): the textbook conditional entropy (EU:321-327) of every
+    user's own (current tile, next tile) pairs over the frames, averaged over the tile counts."""
+    entropy: torch.Tensor            # [U] float64, mean over tile counts; NaN for a user without any pair
+    per_k: Optional[torch.Tensor]    # [K, U] float64
+    pairs: torch.Tensor              # [U] int32 N_u: frames f with the user present in f and f+1
+
+
 def _check(rc: int) -> None:
     if rc == N.VET_OK:
         return
@@ -510,6 +519,27 @@ class Engine:
         acc = self.transition_counts_accumulator()
         self.transition_counts_accumulate(packed, acc)
         return self.transition_counts_finish(acc)
+
+    # -- per-viewer transition entropy ---------------------------------------------------------
+    def user_transitions(self, packed: torch.Tensor, want_per_k: bool = True) -> UserTransitionResult:
+        """Per-viewer transition entropy of packed[F,U,3] (vet_user_transitions): per user and tile count the
+        conditional entropy -sum (n_pc/N_u) log2(n_pc/n_p) of the user's moves from tile p in frame f to tile c in frame
+        f+1, normalised like the textbook mode, and its mean over the tile counts.  One call sees every frame of its
+        users; a user's outputs do not depend on the other users of the call, so user blocks (columns of the video)
+        can be computed separately.  A user without any pair gets NaN.  Call raise_for_flags() to raise for
+        out-of-range coordinates."""
+        p, dt = self._packed(packed)
+        if p.dim() != 3:
+            raise ValueError("packed must be [F, U, 3]")
+        F, U = int(p.shape[0]), int(p.shape[1])
+        K, dev = len(self.tile_counts), self.device
+        out = UserTransitionResult(
+            entropy=torch.empty(U, dtype=torch.float64, device=dev),
+            per_k=torch.empty((K, U), dtype=torch.float64, device=dev) if want_per_k else None,
+            pairs=torch.empty(U, dtype=torch.int32, device=dev))
+        _check(self._lib.vet_user_transitions(self._h, p.data_ptr(), dt, F, U, out.entropy.data_ptr(), _ptr(out.per_k),
+                                              out.pairs.data_ptr(), self._stream()))
+        return out
 
     # -- host-buffer (numpy) variants -----------------------------------------------------
     def spatial_host(self, packed: np.ndarray, want_per_k: bool = True, want_hist0: bool = True,
