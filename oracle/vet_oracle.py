@@ -456,17 +456,20 @@ def cell_luts(W: int, H: int, tile_counts: Sequence[int]) -> List[np.ndarray]:
 
 
 def spatial_analyzer(packed: np.ndarray, W: int, H: int, tile_counts: Sequence[int],
-                     fov_angle=120.0, use_weight=True, power_factor=2.0):
+                     fov_angle=120.0, use_weight=True, power_factor=2.0,
+                     centres: Optional[Sequence[np.ndarray]] = None):
     """SA:129-161 on packed[F,U,3]=(time,2dmu,2dmv); NaN 2dmu/2dmv = missing.
     Returns dict(entropy[F] (mean over tile counts), per_k[K,F], hist0[F,T0],
     assign0[F,U] uint16 (MISSING for absent users)).  A frame without users
-    raises like EU:168-169."""
+    raises like EU:168-169.  `centres` optionally replaces the Fibonacci
+    lattices by arbitrary tile centres (the reference's free functions take any
+    list of vectors)."""
     packed = np.asarray(packed)
     F, U, _ = packed.shape
     px, py, valid = decode(packed[..., 1], packed[..., 2], W, H)
     cv = cell_vectors(W, H)
-    lats = [lattice(n) for n in tile_counts]
-    K = len(tile_counts)
+    lats = [np.asarray(c, dtype=np.float64) for c in centres] if centres is not None else [lattice(n) for n in tile_counts]
+    K = len(lats)
     T0 = len(lats[0])
     per_k = np.empty((K, F), dtype=np.float64)
     hist0 = np.zeros((F, T0), dtype=np.float64)
@@ -489,17 +492,23 @@ def spatial_analyzer(packed: np.ndarray, W: int, H: int, tile_counts: Sequence[i
 
 
 def transition_analyzer(packed: np.ndarray, W: int, H: int, tile_counts: Sequence[int],
-                        mode: str = "literal"):
+                        mode: str = "literal", centres: Optional[Sequence[np.ndarray]] = None):
     """TA:129-172 on packed[F,U,3].  Row r describes frames (r, r+1); users must
     be present in both.  Returns dict(entropy[F-1], per_k[K,F-1],
-    prev_count0[F-1,T0] int32, pairs0[F-1,U,2] uint16)."""
+    prev_count0[F-1,T0] int32, pairs0[F-1,U,2] uint16).  `centres` as in
+    spatial_analyzer."""
     packed = np.asarray(packed)
     F, U, _ = packed.shape
     px, py, valid = decode(packed[..., 1], packed[..., 2], W, H)
     cell = py * (W + 1) + px
-    luts = cell_luts(W, H, tile_counts)
-    Ts = [lattice_size(n) for n in tile_counts]
-    K = len(tile_counts)
+    if centres is not None:
+        cvf = cell_vectors(W, H).reshape(-1, 3)
+        luts = [nearest_tile(cvf, np.asarray(c, dtype=np.float64), chunk=512) for c in centres]
+        Ts = [len(c) for c in centres]
+    else:
+        luts = cell_luts(W, H, tile_counts)
+        Ts = [lattice_size(n) for n in tile_counts]
+    K = len(Ts)
     per_k = np.empty((K, max(F - 1, 0)), dtype=np.float64)
     prev_count0 = np.zeros((max(F - 1, 0), Ts[0]), dtype=np.int32)
     pairs0 = np.full((max(F - 1, 0), U, 2), MISSING, dtype=np.uint16)

@@ -48,17 +48,26 @@ __global__ void k_decode(const TIN* __restrict__ packed, int64_t n, int W, int H
   }
 }
 
+// The unit centres [3 T] of a tile set for the kernels below: copied to shared memory when the launch gave room for
+// them (staged != 0, block-uniform), else read from global memory -- above ~9.6k tiles they do not fit the 227 KB of
+// opt-in shared memory (unit_smem on the host).  The values and so the results are the same either way.
+__device__ __forceinline__ const double* stage_units(const double* __restrict__ unit, int T, double* s_buf, int staged) {
+  if (!staged) return unit;
+  for (int i = threadIdx.x; i < 3 * T; i += blockDim.x) s_buf[i] = unit[i];
+  __syncthreads();
+  return s_buf;
+}
+
 // Stage 2: brute-force exact nearest tile.  Four lanes share one vector: lane j
 // scans tiles j, j+4, ... keeping the first strict maximum of the fp64 dot
 // (== first minimum of arccos, EU:104); the four partial winners are merged with
 // two shuffle steps, larger dot first and lower tile index on ties.  Unit tile
-// centres sit in shared memory (broadcast reads).
+// centres sit in shared memory (broadcast reads) where they fit (stage_units).
 template <typename TOUT>
 __global__ void k_nearest(const double* __restrict__ vec, int64_t n, const double* __restrict__ unit, int T,
-                          TOUT* __restrict__ idx_out) {
-  extern __shared__ double s_unit[];
-  for (int i = threadIdx.x; i < 3 * T; i += blockDim.x) s_unit[i] = unit[i];
-  __syncthreads();
+                          TOUT* __restrict__ idx_out, int staged) {
+  extern __shared__ double s_buf[];
+  const double* s_unit = stage_units(unit, T, s_buf, staged);
   const int sub = threadIdx.x & 3;
   const int64_t per_block = blockDim.x >> 2;
   const int64_t rounds = (n + per_block - 1) / per_block;
@@ -95,12 +104,11 @@ __global__ void k_nearest(const double* __restrict__ vec, int64_t n, const doubl
   }
 }
 
-// calculate_tile_weights (EU:108-144), dense rows for arbitrary vectors.
+// calculate_tile_weights (EU:108-144), dense rows for arbitrary vectors (unit centres as in k_nearest).
 __global__ void k_tile_weights(const double* __restrict__ vec, int64_t n, const double* __restrict__ unit, int T,
-                               double max_d, double pf, int use_weight, double* __restrict__ w_out) {
-  extern __shared__ double s_unit[];
-  for (int i = threadIdx.x; i < 3 * T; i += blockDim.x) s_unit[i] = unit[i];
-  __syncthreads();
+                               double max_d, double pf, int use_weight, double* __restrict__ w_out, int staged) {
+  extern __shared__ double s_buf[];
+  const double* s_unit = stage_units(unit, T, s_buf, staged);
   // one warp per vector
   const int lane = threadIdx.x & 31;
   const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
