@@ -89,6 +89,13 @@ def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
 
+def _mode(mode: str) -> int:
+    """VET_TRANSITION_* code of a transition mode name."""
+    if mode not in ("literal", "textbook"):
+        raise ValueError("mode must be 'literal' or 'textbook'")
+    return N.VET_TRANSITION_LITERAL if mode == "literal" else N.VET_TRANSITION_TEXTBOOK
+
+
 class Engine:
     """One native handle.  Not thread-safe per instance; use one per thread/stream."""
 
@@ -182,6 +189,31 @@ class Engine:
         if packed.shape[-1] != 3:
             raise ValueError("packed must have shape [..., 3] = (time, 2dmu, 2dmv)")
         return packed.contiguous(), (N.VET_F32 if packed.dtype == torch.float32 else N.VET_F64)
+
+    def _frames(self, packed: torch.Tensor) -> Tuple[torch.Tensor, int, int, int]:
+        """_packed for the [F, U, 3] inputs of the frame-level calls -> (packed, dtype code, F, U)."""
+        p, dt = self._packed(packed)
+        if p.dim() != 3:
+            raise ValueError("packed must be [F, U, 3]")
+        return p, dt, int(p.shape[0]), int(p.shape[1])
+
+    def _spatial_result(self, F: int, U: int, want_per_k: bool, want_hist0: bool, want_assign0: bool) -> SpatialResult:
+        K, T0, dev = len(self.tile_counts), self.num_tiles[0], self.device
+        return SpatialResult(
+            entropy=torch.empty(F, dtype=torch.float64, device=dev),
+            per_k=torch.empty((K, F), dtype=torch.float64, device=dev) if want_per_k else None,
+            hist0=torch.empty((F, T0), dtype=torch.float64, device=dev) if want_hist0 else None,
+            assign0=torch.empty((F, U), dtype=torch.uint16, device=dev) if want_assign0 else None)
+
+    def _transition_result(self, F: int, U: int, want_per_k: bool, want_prev_count0: bool,
+                           want_pairs0: bool) -> TransitionResult:
+        R = max(F - 1, 0)
+        K, T0, dev = len(self.tile_counts), self.num_tiles[0], self.device
+        return TransitionResult(
+            entropy=torch.empty(R, dtype=torch.float64, device=dev),
+            per_k=torch.empty((K, R), dtype=torch.float64, device=dev) if want_per_k else None,
+            prev_count0=torch.empty((R, T0), dtype=torch.int32, device=dev) if want_prev_count0 else None,
+            pairs0=torch.empty((R, U, 2), dtype=torch.uint16, device=dev) if want_pairs0 else None)
 
     def set_option(self, name: str, value) -> None:
         """vet_set_option: pins a kernel choice of this handle, e.g. set_option("weighted_kernel", "i8")
@@ -295,12 +327,7 @@ class Engine:
         if v.dim() != 3 or v.shape[-1] != 3:
             raise ValueError("vectors must be [F, U, 3]")
         F, U = int(v.shape[0]), int(v.shape[1])
-        K, T0, dev = len(self.tile_counts), self.num_tiles[0], self.device
-        out = SpatialResult(
-            entropy=torch.empty(F, dtype=torch.float64, device=dev),
-            per_k=torch.empty((K, F), dtype=torch.float64, device=dev) if want_per_k else None,
-            hist0=torch.empty((F, T0), dtype=torch.float64, device=dev) if want_hist0 else None,
-            assign0=torch.empty((F, U), dtype=torch.uint16, device=dev) if want_assign0 else None)
+        out = self._spatial_result(F, U, want_per_k, want_hist0, want_assign0)
         _check(self._lib.vet_spatial_vectors(self._h, v.data_ptr(), F, U, out.entropy.data_ptr(), _ptr(out.per_k),
                                              _ptr(out.hist0), _ptr(out.assign0), self._stream()))
         return out
@@ -311,17 +338,9 @@ class Engine:
         v = vectors.to(device=self.device, dtype=torch.float64).contiguous()
         if v.dim() != 3 or v.shape[-1] != 3:
             raise ValueError("vectors must be [F, U, 3]")
-        if mode not in ("literal", "textbook"):
-            raise ValueError("mode must be 'literal' or 'textbook'")
+        m = _mode(mode)
         F, U = int(v.shape[0]), int(v.shape[1])
-        R = max(F - 1, 0)
-        K, T0, dev = len(self.tile_counts), self.num_tiles[0], self.device
-        out = TransitionResult(
-            entropy=torch.empty(R, dtype=torch.float64, device=dev),
-            per_k=torch.empty((K, R), dtype=torch.float64, device=dev) if want_per_k else None,
-            prev_count0=torch.empty((R, T0), dtype=torch.int32, device=dev) if want_prev_count0 else None,
-            pairs0=torch.empty((R, U, 2), dtype=torch.uint16, device=dev) if want_pairs0 else None)
-        m = N.VET_TRANSITION_LITERAL if mode == "literal" else N.VET_TRANSITION_TEXTBOOK
+        out = self._transition_result(F, U, want_per_k, want_prev_count0, want_pairs0)
         _check(self._lib.vet_transition_vectors(self._h, v.data_ptr(), F, U, out.entropy.data_ptr(), _ptr(out.per_k),
                                                 _ptr(out.prev_count0), _ptr(out.pairs0), m, self._stream()))
         return out
@@ -346,18 +365,9 @@ class Engine:
     # -- stages 1-3 fused -----------------------------------------------------------
     def spatial(self, packed: torch.Tensor, want_per_k: bool = True, want_hist0: bool = True,
                 want_assign0: bool = True, out: Optional[SpatialResult] = None) -> SpatialResult:
-        p, dt = self._packed(packed)
-        if p.dim() != 3:
-            raise ValueError("packed must be [F, U, 3]")
-        F, U = int(p.shape[0]), int(p.shape[1])
-        K, T0 = len(self.tile_counts), self.num_tiles[0]
+        p, dt, F, U = self._frames(packed)
         if out is None:
-            dev = self.device
-            out = SpatialResult(
-                entropy=torch.empty(F, dtype=torch.float64, device=dev),
-                per_k=torch.empty((K, F), dtype=torch.float64, device=dev) if want_per_k else None,
-                hist0=torch.empty((F, T0), dtype=torch.float64, device=dev) if want_hist0 else None,
-                assign0=torch.empty((F, U), dtype=torch.uint16, device=dev) if want_assign0 else None)
+            out = self._spatial_result(F, U, want_per_k, want_hist0, want_assign0)
         _check(self._lib.vet_spatial(self._h, p.data_ptr(), dt, F, U, out.entropy.data_ptr(), _ptr(out.per_k),
                                      _ptr(out.hist0), _ptr(out.assign0), self._stream()))
         return out
@@ -366,22 +376,10 @@ class Engine:
     def transition(self, packed: torch.Tensor, mode: str = "literal", want_per_k: bool = True,
                    want_prev_count0: bool = True, want_pairs0: bool = True,
                    out: Optional[TransitionResult] = None) -> TransitionResult:
-        p, dt = self._packed(packed)
-        if p.dim() != 3:
-            raise ValueError("packed must be [F, U, 3]")
-        if mode not in ("literal", "textbook"):
-            raise ValueError("mode must be 'literal' or 'textbook'")
-        F, U = int(p.shape[0]), int(p.shape[1])
-        R = max(F - 1, 0)
-        K, T0 = len(self.tile_counts), self.num_tiles[0]
+        p, dt, F, U = self._frames(packed)
+        m = _mode(mode)
         if out is None:
-            dev = self.device
-            out = TransitionResult(
-                entropy=torch.empty(R, dtype=torch.float64, device=dev),
-                per_k=torch.empty((K, R), dtype=torch.float64, device=dev) if want_per_k else None,
-                prev_count0=torch.empty((R, T0), dtype=torch.int32, device=dev) if want_prev_count0 else None,
-                pairs0=torch.empty((R, U, 2), dtype=torch.uint16, device=dev) if want_pairs0 else None)
-        m = N.VET_TRANSITION_LITERAL if mode == "literal" else N.VET_TRANSITION_TEXTBOOK
+            out = self._transition_result(F, U, want_per_k, want_prev_count0, want_pairs0)
         _check(self._lib.vet_transition(self._h, p.data_ptr(), dt, F, U, out.entropy.data_ptr(), _ptr(out.per_k),
                                         _ptr(out.prev_count0), _ptr(out.pairs0), m, self._stream()))
         return out
@@ -392,25 +390,10 @@ class Engine:
                 want_pairs0: bool = True) -> Tuple[SpatialResult, TransitionResult]:
         """SpatialEntropyAnalyzer.compute_entropy and TransitionEntropyAnalyzer.compute_entropy on
         the same packed tensor with a single read of the input (vet_analyze)."""
-        p, dt = self._packed(packed)
-        if p.dim() != 3:
-            raise ValueError("packed must be [F, U, 3]")
-        if mode not in ("literal", "textbook"):
-            raise ValueError("mode must be 'literal' or 'textbook'")
-        F, U = int(p.shape[0]), int(p.shape[1])
-        R = max(F - 1, 0)
-        K, T0, dev = len(self.tile_counts), self.num_tiles[0], self.device
-        sp = SpatialResult(
-            entropy=torch.empty(F, dtype=torch.float64, device=dev),
-            per_k=torch.empty((K, F), dtype=torch.float64, device=dev) if want_per_k else None,
-            hist0=torch.empty((F, T0), dtype=torch.float64, device=dev) if want_hist0 else None,
-            assign0=torch.empty((F, U), dtype=torch.uint16, device=dev) if want_assign0 else None)
-        tr = TransitionResult(
-            entropy=torch.empty(R, dtype=torch.float64, device=dev),
-            per_k=torch.empty((K, R), dtype=torch.float64, device=dev) if want_per_k else None,
-            prev_count0=torch.empty((R, T0), dtype=torch.int32, device=dev) if want_prev_count0 else None,
-            pairs0=torch.empty((R, U, 2), dtype=torch.uint16, device=dev) if want_pairs0 else None)
-        m = N.VET_TRANSITION_LITERAL if mode == "literal" else N.VET_TRANSITION_TEXTBOOK
+        p, dt, F, U = self._frames(packed)
+        m = _mode(mode)
+        sp = self._spatial_result(F, U, want_per_k, want_hist0, want_assign0)
+        tr = self._transition_result(F, U, want_per_k, want_prev_count0, want_pairs0)
         _check(self._lib.vet_analyze(self._h, p.data_ptr(), dt, F, U, sp.entropy.data_ptr(), _ptr(sp.per_k), _ptr(sp.hist0),
                                      _ptr(sp.assign0), tr.entropy.data_ptr(), _ptr(tr.per_k), _ptr(tr.prev_count0),
                                      _ptr(tr.pairs0), m, self._stream()))
@@ -435,10 +418,7 @@ class Engine:
         """Adds the frames of packed[F,U,3] into acc (vet_users_accumulate).  total_frames is the frame count of the
         whole video: every batch (and every rank) of one video must pass the same value, which fixes the fixed-point
         scale of the weights -- then any batching or frame order gives the same bits."""
-        p, dt = self._packed(packed)
-        if p.dim() != 3:
-            raise ValueError("packed must be [F, U, 3]")
-        F, U = int(p.shape[0]), int(p.shape[1])
+        p, dt, F, U = self._frames(packed)
         self._check_acc(acc, U)
         if int(total_frames) < max(F, 1):
             raise ValueError(f"total_frames ({total_frames}) must be >= 1 and >= the frames of packed ({F})")
@@ -465,10 +445,7 @@ class Engine:
         """Per-viewer exploration entropy of packed[F,U,3]: compute_spatial_entropy (EU:147-211) of every user's
         present samples over the frames, averaged over the tile counts (SA:142-156).  A user without any sample
         gets NaN and a zero histogram row.  Call raise_for_flags() to raise for out-of-range coordinates."""
-        p, _ = self._packed(packed)
-        if p.dim() != 3:
-            raise ValueError("packed must be [F, U, 3]")
-        F, U = int(p.shape[0]), int(p.shape[1])
+        p, _, F, U = self._frames(packed)
         acc = self.user_accumulator(U)
         self.users_accumulate(p, acc, max(F, 1))
         return self.users_finish(acc, max(F, 1), want_per_k, want_hist0)
@@ -489,12 +466,9 @@ class Engine:
     def transition_counts_accumulate(self, packed: torch.Tensor, acc: torch.Tensor) -> None:
         """Adds the (f, f+1) frame pairs of packed[F,U,3] into acc (vet_transition_counts_accumulate).  Batches that
         overlap by one frame add up to the whole video, in any batching and order, with the same bits."""
-        p, dt = self._packed(packed)
-        if p.dim() != 3:
-            raise ValueError("packed must be [F, U, 3]")
+        p, dt, F, U = self._frames(packed)
         self._check_tc_acc(acc)
-        _check(self._lib.vet_transition_counts_accumulate(self._h, p.data_ptr(), dt, int(p.shape[0]), int(p.shape[1]),
-                                                          acc.data_ptr(), self._stream()))
+        _check(self._lib.vet_transition_counts_accumulate(self._h, p.data_ptr(), dt, F, U, acc.data_ptr(), self._stream()))
 
     def transition_counts_finish(self, acc: torch.Tensor) -> TransitionCountsResult:
         """Pooled conditional entropy of the finished counts (vet_transition_counts_finish); `counts` are views of acc.
@@ -528,10 +502,7 @@ class Engine:
         users; a user's outputs do not depend on the other users of the call, so user blocks (columns of the video)
         can be computed separately.  A user without any pair gets NaN.  Call raise_for_flags() to raise for
         out-of-range coordinates."""
-        p, dt = self._packed(packed)
-        if p.dim() != 3:
-            raise ValueError("packed must be [F, U, 3]")
-        F, U = int(p.shape[0]), int(p.shape[1])
+        p, dt, F, U = self._frames(packed)
         K, dev = len(self.tile_counts), self.device
         out = UserTransitionResult(
             entropy=torch.empty(U, dtype=torch.float64, device=dev),
@@ -552,16 +523,11 @@ class Engine:
         arr, dt, F, U = _host_packed(packed)
         self._host_layout(arr)
         K, T0 = len(self.tile_counts), self.num_tiles[0]
-        key = (F, U, want_per_k, want_hist0, want_assign0)
-        bufs = self._host_out.get(key) if reuse_buffers else None
-        if bufs is None:
-            bufs = (_pinned((F,), np.float64),
-                    _pinned((K, F), np.float64) if want_per_k else None,
-                    _pinned((F, T0), np.float64) if want_hist0 else None,
-                    _pinned((F, U), np.uint16) if want_assign0 else None)
-            if reuse_buffers:
-                self._host_out = {key: bufs}
-        ent, per_k, hist0, assign0 = bufs
+        ent, per_k, hist0, assign0 = self._host_buffers(
+            ("sp", F, U, want_per_k, want_hist0, want_assign0),
+            lambda: (_pinned((F,), np.float64), _pinned((K, F), np.float64) if want_per_k else None,
+                     _pinned((F, T0), np.float64) if want_hist0 else None,
+                     _pinned((F, U), np.uint16) if want_assign0 else None), reuse_buffers)
         _check(self._lib.vet_spatial_host(self._h, _host_ptr(arr), dt, F, U, ent.ctypes.data, _np_ptr(per_k),
                                           _np_ptr(hist0), _np_ptr(assign0)))
         return dict(entropy=ent, per_k=per_k, hist0=hist0, assign0=assign0)
@@ -588,8 +554,7 @@ class Engine:
         one-frame halo, upload | kernels | download on three streams; results in page-locked memory."""
         arr, dt, F, U = _host_packed(packed)
         self._host_layout(arr)
-        if mode not in ("literal", "textbook"):
-            raise ValueError("mode must be 'literal' or 'textbook'")
+        m = _mode(mode)
         R = max(F - 1, 0)
         K, T0 = len(self.tile_counts), self.num_tiles[0]
         ent, per_k, pc, pairs = self._host_buffers(
@@ -597,7 +562,6 @@ class Engine:
             lambda: (_pinned((R,), np.float64), _pinned((K, R), np.float64) if want_per_k else None,
                      _pinned((R, T0), np.int32) if want_prev_count0 else None,
                      _pinned((R, U, 2), np.uint16) if want_pairs0 else None), reuse_buffers)
-        m = N.VET_TRANSITION_LITERAL if mode == "literal" else N.VET_TRANSITION_TEXTBOOK
         _check(self._lib.vet_transition_host(self._h, _host_ptr(arr), dt, F, U, ent.ctypes.data, _np_ptr(per_k),
                                              _np_ptr(pc), _np_ptr(pairs), m))
         return dict(entropy=ent, per_k=per_k, prev_count0=pc, pairs0=pairs)
@@ -609,8 +573,7 @@ class Engine:
         dicts of numpy arrays like spatial_host / transition_host."""
         arr, dt, F, U = _host_packed(packed)
         self._host_layout(arr)
-        if mode not in ("literal", "textbook"):
-            raise ValueError("mode must be 'literal' or 'textbook'")
+        m = _mode(mode)
         R = max(F - 1, 0)
         K, T0 = len(self.tile_counts), self.num_tiles[0]
         bufs = self._host_buffers(
@@ -622,7 +585,6 @@ class Engine:
                      _pinned((R, T0), np.int32) if want_prev_count0 else None,
                      _pinned((R, U, 2), np.uint16) if want_pairs0 else None), reuse_buffers)
         ent, per_k, hist0, assign0, tent, tper_k, pc, pairs = bufs
-        m = N.VET_TRANSITION_LITERAL if mode == "literal" else N.VET_TRANSITION_TEXTBOOK
         _check(self._lib.vet_analyze_host(self._h, _host_ptr(arr), dt, F, U, ent.ctypes.data, _np_ptr(per_k), _np_ptr(hist0),
                                           _np_ptr(assign0), tent.ctypes.data, _np_ptr(tper_k), _np_ptr(pc), _np_ptr(pairs), m))
         return (dict(entropy=ent, per_k=per_k, hist0=hist0, assign0=assign0),
